@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- transition frames/sec of the branch-tree denoising hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one ``BlendingEngine.run_transition()`` of the selected BASELINE.json config (default: configs[1], the
@@ -16,6 +16,8 @@ Prints ONE JSON line (rank 0).  ``value`` = frames/s with the conditioning alrea
 the device; ``e2e`` = the same through the public API (set_prompt1/2 -> run_transition -> PIL frames), host<->device
 copies timed.  ``fingerprint`` = sha1 over the tree (tree_fracts, tree_idx_injection, every branch's final latents):
 equal fingerprints across --gpus 1/2/4/8 mean the sharded run built exactly the single-GPU tree.
+``--dump-outputs DIR`` writes the frames, final latents and fractions of the last timed step as .npy files, so that
+two builds can be compared output for output on the same seeded inputs.
 ``--impl reference`` times the CPU oracle (a port of the reference path: diffusers / lpips are not installable
 here) on the host cores this process may use.
 """
@@ -347,6 +349,27 @@ def tree_fingerprint(be):
     return h.hexdigest()
 
 
+DUMP_FRAME_VALUES = 1 << 23     # 32 MB of float32 frame samples; the final latents add at most 8 MB (config 3)
+
+
+def dump_outputs(out_dir, frames, be):
+    """Write what the last timed step computed as .npy files under ``out_dir``:
+    ``frames`` float32 [n_frames, k]: the returned uint8 RGB frames at k pixel-channel positions drawn once from a
+    fixed seed (the same positions in every frame; all of them when the frames are small enough),
+    ``final_latents`` float32 [n_branches, ...]: every branch's final latents in tree order,
+    ``tree_fracts`` float64 [n_branches]: the branches' mixing fractions."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    fr = torch.stack(frames).reshape(len(frames), -1)
+    k = min(fr.shape[1], DUMP_FRAME_VALUES // len(frames))
+    idx = np.sort(np.random.default_rng(0).choice(fr.shape[1], k, replace=False))
+    np.save(os.path.join(out_dir, "frames.npy"), fr[:, torch.from_numpy(idx).to(fr.device)].float().cpu().numpy())
+    finals = torch.stack([t[-1] for t in be.tree_latents], 0)
+    np.save(os.path.join(out_dir, "final_latents.npy"), finals.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "tree_fracts.npy"), np.asarray(be.tree_fracts, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     rank, local_rank, world = dist_env()
@@ -404,15 +427,18 @@ def run_ours(args):
             ms = float(t)
         return ms / 1e3, n
 
+    step_frames = []        # the frames returned in the latest step
+
     def one_job(api):
         """One bench step.  Configs 2/3/5: one transition.  Config 4: the 8-prompt loop (7 transitions)."""
         be.output_device_frames = not api
+        step_frames.clear()
         if args.config != 4:
             if api:
                 be.set_prompt1(PROMPTS[0])
                 be.set_prompt2(PROMPTS[1])
-            return len(be.run_transition(fixed_seeds=list(cfg["seeds"])))
-        n = 0
+            step_frames.extend(be.run_transition(fixed_seeds=list(cfg["seeds"])))
+            return len(step_frames)
         for i in range(len(PROMPTS_MULTI) - 1):
             if i == 0:
                 be.set_prompt1(PROMPTS_MULTI[0])
@@ -420,19 +446,23 @@ def run_ours(args):
             else:
                 be.swap_forward()
                 be.set_prompt2(PROMPTS_MULTI[i + 1])
-            n += len(be.run_transition(recycle_img1=i > 0, fixed_seeds=[420 + i, 421 + i]))
-        return n
+            step_frames.extend(be.run_transition(recycle_img1=i > 0, fixed_seeds=[420 + i, 421 + i]))
+        return len(step_frames)
 
     for _ in range(max(args.warmup, 0)):
         one_job(False)
     sampler = ClockSampler(local_rank)
     sampler.start()
-    ops.LAUNCHES[0] = 0
-    sec, frames = timed(lambda: one_job(False), args.steps)
-    launches = ops.LAUNCHES[0]
-    clocks = sampler.stop()
+    try:
+        ops.LAUNCHES[0] = 0
+        sec, frames = timed(lambda: one_job(False), args.steps)
+        launches = ops.LAUNCHES[0]
+    finally:
+        clocks = sampler.stop()
     fps = frames / sec
     fingerprint = tree_fingerprint(be)          # of the last timed transition (identical every step: fixed seeds)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_frames, be)
     stems_run = [int(v) for v in be.list_nmb_stems]
     # e2e through the public API with host buffers
     one_job(True)
@@ -545,7 +575,13 @@ def main():
     ap.add_argument("--t-compute", type=float, default=6.0,
                     help="config 4: t_compute_max_allowed per transition (the reference default is 20 s)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,11 +1,12 @@
-"""Generate golden fixtures by IMPORTING THE REFERENCE (run in the build container
-only; /root/reference does not exist on the GPU box, the tests read the
-committed fixture files).
+"""Generate golden fixtures by IMPORTING THE REFERENCE (needs a checkout of
+lunarring/latentblending; the tests only read the committed fixture files).
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <path to the latentblending checkout>
 
 * slerp.npz      -- latentblending/utils.py interpolate_spherical / interpolate_linear
                     outputs on seeded inputs (fp16 and fp32, several fracts incl. 0/1).
+                    The tests rebuild the seeded inputs with slerp_cases(), so only the
+                    reference's outputs and a checksum of the inputs are stored.
 * tree.json      -- the reference BlendingEngine host logic (run_transition,
                     get_mixing_parameters, insert_into_tree, compute_latents_mix
                     coefficient schedules, set_guidance_mid_dampening,
@@ -15,6 +16,7 @@ The reference's third-party imports (diffusers, lpips, lunar_tools) are absent
 here; they are stubbed with empty modules -- none of their code is on the host
 logic exercised.
 """
+import hashlib
 import json
 import os
 import sys
@@ -25,7 +27,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
-REF = "/root/reference"
+SLERP_FIXTURE = os.path.join(HERE, "slerp.npz")
 
 
 def _stub(name, **attrs):
@@ -36,7 +38,7 @@ def _stub(name, **attrs):
     return m
 
 
-def import_reference():
+def import_reference(ref_dir):
     _stub("lpips", LPIPS=object)
     _stub("lunar_tools", MovieSaver=object, fill_up_frames_linear_interpolation=None)
     _stub("diffusers", DiffusionPipeline=object, StableDiffusionControlNetPipeline=object, ControlNetModel=object)
@@ -46,31 +48,54 @@ def import_reference():
     _stub("diffusers.pipelines")
     _stub("diffusers.pipelines.stable_diffusion_xl")
     _stub("diffusers.pipelines.stable_diffusion_xl.pipeline_stable_diffusion_xl", retrieve_timesteps=None)
-    sys.path.insert(0, REF)
+    sys.path.insert(0, ref_dir)
     import latentblending.utils as ref_utils
     import latentblending.blending_engine as ref_engine
     return ref_utils, ref_engine
 
 
-def golden_slerp(ref_utils):
-    out = {}
+def slerp_cases():
+    """The seeded (p0, p1, fract) inputs of slerp.npz and the generator they leave behind (it then draws the
+    interpolate_linear inputs)."""
     g = torch.Generator().manual_seed(1234)
-    cases = []
+    shapes = []
     for n, dt in ((64, torch.float16), (4 * 16 * 16, torch.float16), (4 * 64 * 64, torch.float16),
                   (4 * 128 * 128, torch.float16), (777, torch.float32)):
         for f in (0.0, 0.25, 0.5, 0.3141, 1.0):
-            cases.append((n, dt, f))
-    for k, (n, dt, f) in enumerate(cases):
+            shapes.append((n, dt, f))
+    cases = []
+    for k, (n, dt, f) in enumerate(shapes):
         p0 = (torch.randn(n, generator=g) * (1 + k % 3)).to(dt)
         p1 = (torch.randn(n, generator=g) * 2).to(dt)
         if k % 7 == 3:
             p1 = (p0.float() * 1.5).to(dt)          # parallel vectors -> exercises the 1e-7 clamp
-        r = ref_utils.interpolate_spherical(p0, p1, f)
-        out[f"p0_{k}"] = p0.numpy()
-        out[f"p1_{k}"] = p1.numpy()
-        out[f"f_{k}"] = np.float64(f)
-        out[f"out_{k}"] = r.numpy()
+        cases.append((p0, p1, f))
+    return cases, g
+
+
+def slerp_inputs_sha1(cases):
+    h = hashlib.sha1()
+    for p0, p1, f in cases:
+        h.update(p0.numpy().tobytes())
+        h.update(p1.numpy().tobytes())
+        h.update(np.float64(f).tobytes())
+    return h.hexdigest()
+
+
+def load_slerp_golden():
+    """(p0, p1, fract, reference output) of every slerp case."""
+    z = np.load(SLERP_FIXTURE)
+    cases, _ = slerp_cases()
+    assert len(cases) == int(z["n_cases"])
+    assert slerp_inputs_sha1(cases) == str(z["inputs_sha1"]), "seeded slerp inputs drifted from the fixture's"
+    return [(p0, p1, f, torch.from_numpy(z[f"out_{k}"])) for k, (p0, p1, f) in enumerate(cases)]
+
+
+def golden_slerp(ref_utils):
+    cases, g = slerp_cases()
+    out = {f"out_{k}": ref_utils.interpolate_spherical(p0, p1, f).numpy() for k, (p0, p1, f) in enumerate(cases)}
     out["n_cases"] = np.int64(len(cases))
+    out["inputs_sha1"] = np.array(slerp_inputs_sha1(cases))
     # interpolate_linear on tensors and uint8 frames
     a = torch.randn(1, 77, 64, generator=g).half()
     b = torch.randn(1, 77, 64, generator=g).half()
@@ -80,7 +105,7 @@ def golden_slerp(ref_utils):
     ib = (torch.rand(8, 8, 3, generator=g) * 255).byte().numpy()
     out["lin_ia"], out["lin_ib"] = ia, ib
     out["lin_iout"] = ref_utils.interpolate_linear(ia, ib, 0.6)
-    np.savez_compressed(os.path.join(HERE, "slerp.npz"), **out)
+    np.savez_compressed(SLERP_FIXTURE, **out)
     print("slerp.npz:", len(cases), "cases")
 
 
@@ -177,6 +202,8 @@ def golden_tree(ref_engine):
 
 
 if __name__ == "__main__":
-    ref_utils, ref_engine = import_reference()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    ref_utils, ref_engine = import_reference(sys.argv[1])
     golden_slerp(ref_utils)
     golden_tree(ref_engine)

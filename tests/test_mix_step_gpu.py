@@ -13,12 +13,9 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 def test_slerp_golden_bit_exact():
     from latentblending_b200 import utils
-    z = np.load(os.path.join(GOLD, "slerp.npz"))
-    for k in range(int(z["n_cases"])):
-        p0 = torch.from_numpy(z[f"p0_{k}"]).cuda()
-        p1 = torch.from_numpy(z[f"p1_{k}"]).cuda()
-        out = utils.interpolate_spherical(p0, p1, float(z[f"f_{k}"])).cpu()
-        ref = torch.from_numpy(z[f"out_{k}"])
+    from make_golden import load_slerp_golden
+    for k, (p0, p1, f, ref) in enumerate(load_slerp_golden()):
+        out = utils.interpolate_spherical(p0.cuda(), p1.cuda(), f).cpu()
         assert out.dtype == ref.dtype
         assert torch.equal(out, ref), f"case {k}: {(out != ref).sum().item()} mismatches"
 

@@ -17,11 +17,9 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def test_slerp_matches_reference_golden():
-    z = np.load(os.path.join(GOLD, "slerp.npz"))
-    for k in range(int(z["n_cases"])):
-        p0, p1 = torch.from_numpy(z[f"p0_{k}"]), torch.from_numpy(z[f"p1_{k}"])
-        out = mixing.interpolate_spherical(p0, p1, float(z[f"f_{k}"]))
-        ref = torch.from_numpy(z[f"out_{k}"])
+    from make_golden import load_slerp_golden
+    for k, (p0, p1, f, ref) in enumerate(load_slerp_golden()):
+        out = mixing.interpolate_spherical(p0, p1, f)
         assert out.dtype == ref.dtype
         assert torch.equal(out, ref), f"case {k}"
 
